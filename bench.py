@@ -344,9 +344,12 @@ def run_ours(args):
     launches = ops.launch_count() - l0
     W = max(args.warmup, 3)
     single = None
+    dumped = None
     if not pipelined:
         dr = lambda: slots[0].gather.drain(slots[0].index)
         total_ms = timed(slots[0].step_resident, args.steps, W, dr)
+        if args.dump_outputs:
+            dumped = host_outputs(slots[0].outputs)
         e2e_blob_ms = timed(slots[0].step_e2e_blob, args.steps, 1, dr)
         if use_graph:
             slots[0].build_e2e_graph()
@@ -358,6 +361,8 @@ def run_ours(args):
                   "schedule": "latency: left/right chains, RPN levels and box head forked onto a second stream",
                   "l2": "256 MB flush between timed iterations"}
         total_ms = timed_pipelined("step_resident", args.steps, W + n_inflight)
+        if args.dump_outputs:
+            dumped = host_outputs(slots[(args.steps - 1) % n_inflight].outputs)     # the slot of the last step
         e2e_blob_ms = timed_pipelined("step_e2e_blob", args.steps, W + n_inflight)
         if use_graph:
             for sl in slots:
@@ -422,6 +427,10 @@ def run_ours(args):
         dist.destroy_process_group()
     if rank != 0:
         return
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     out = {
         "metric": "stereo pairs/sec (1242x375)", "value": round(value, 3), "unit": "pairs/s", "n_gpus": world,
         "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": round(ms_per_step, 3),
@@ -464,6 +473,19 @@ def run_ours(args):
     if parity is not None:
         out["parity"] = parity
     print(json.dumps(out))
+
+
+def host_outputs(outputs):
+    """what StereoPipeline.step returned -- (record, keep, nkeep, status, best_dis) of MB pairs -- as host float32 /
+    float64 arrays.  Entries of `keep` past `nkeep` are left unwritten by the NMS kernel and are set to -1 here."""
+    rec, keep, nkeep, st, dis = outputs
+    torch.cuda.synchronize()
+    nkeep = nkeep.cpu().numpy()
+    keep = keep.cpu().numpy().astype(np.float64)
+    for b, n in enumerate(nkeep):
+        keep[b, n:] = -1
+    return {"record": rec.float().cpu().numpy(), "keep": keep, "nkeep": nkeep.astype(np.float64),
+            "status": torch.stack(st).float().cpu().numpy(), "best_dis": torch.stack(dis).float().cpu().numpy()}
 
 
 def conv_time_per_step(pipe, iml, imr):
@@ -649,7 +671,7 @@ def run_reference(args):
     for _ in range(min(args.warmup, 1)):
         cpu_port_step(sd, left, right, wcrop, rois3d, calib)
     tot = 0.0
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     for _ in range(steps):
         tot += cpu_port_step(sd, left, right, wcrop, rois3d, calib)
     value = steps * (wcrop / W_NET) / tot
@@ -683,7 +705,13 @@ def main():
                     help="peer exchange: 1 = pipelined (a step collects the previous step's records), 0 = same step")
     ap.add_argument("--inflight", type=int, default=int(os.environ.get("SB_INFLIGHT", "3")),
                     help="independent pairs in flight per GPU (each batch-1, own stream + CUDA graph)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline path returned in its last step (record, "
+                         "keep, nkeep, status, best_dis of rank 0) as DIR/<name>.npy; the inputs are seeded, so two "
+                         "builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

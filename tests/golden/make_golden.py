@@ -179,11 +179,61 @@ def train_goldens():
     np.savez_compressed(os.path.join(HERE, "train_targets.npz"), **out)
 
 
+def ref_kernel_goldens(out_dir=HERE):
+    """(12) outputs of the reference's own CUDA kernels (nms_cuda_compute, ROIAlignForwardLaucher,
+    ROIAlignBackwardLaucher), compiled unmodified for sm_100a by oracle/build.py build_ref(), on the seeded inputs of
+    tests/test_gpu_ops.py.  Needs a GPU and oracle/_ref/libref_ops.so:
+
+        python tests/golden/make_golden.py ref_kernels [OUT_DIR]
+
+    The RoIAlign outputs are stored at a fixed seeded sample of positions (plus every output of the edge-case RoIs 0
+    and 1) and as (sum, sum of magnitudes) over the whole array, which keeps the fixture small."""
+    import ctypes
+    from oracle import build as ob
+    sys.path.insert(0, os.path.join(HERE, ".."))
+    from test_gpu_ops import NMS_REF_CASES, rand_dets, roi_align_ref_inputs
+    so = ob.build_ref()
+    assert so is not None, "oracle/_ref/libref_ops.so not built (needs the reference's sources)"
+    lib = ctypes.CDLL(so)
+    p = lambda t: ctypes.c_void_p(t.data_ptr())
+    out = {}
+    for n, seed in NMS_REF_CASES:
+        d = torch.from_numpy(rand_dets(n, seed)).cuda()
+        keep = torch.zeros(n, dtype=torch.int32, device="cuda")
+        num = torch.zeros(1, dtype=torch.int32, device="cuda")
+        torch.cuda.synchronize()
+        lib.nms_cuda_compute(p(keep), p(num), p(d), n, 5, ctypes.c_float(0.7))
+        torch.cuda.synchronize()
+        out["nms_keep_%d_%d" % (n, seed)] = keep[:int(num[0])].cpu().numpy()
+    feat, rois, top = roi_align_ref_inputs()
+    f, r, t = (torch.from_numpy(a).cuda() for a in (feat, rois, top))
+    R, C, H, W, P = rois.shape[0], feat.shape[1], feat.shape[2], feat.shape[3], 8
+    fwd = torch.zeros(R, C, P, P, device="cuda")
+    bwd = torch.zeros(1, C, H, W, device="cuda")
+    torch.cuda.synchronize()
+    lib.ROIAlignForwardLaucher(p(f), ctypes.c_float(0.25), R, H, W, C, P, P, p(r), p(fwd), ctypes.c_void_p(0))
+    lib.ROIAlignBackwardLaucher(p(t), ctypes.c_float(0.25), 1, R, H, W, C, P, P, p(r), p(bwd), ctypes.c_void_p(0))
+    torch.cuda.synchronize()
+    fwd, bwd = fwd.cpu().numpy().reshape(-1), bwd.cpu().numpy().reshape(-1)
+    rs = np.random.RandomState(12)
+    edge = 2 * C * P * P                                 # RoI 0 (all zero) and RoI 1 (extrapolation band)
+    fidx = np.concatenate([np.arange(edge), np.sort(rs.choice(np.arange(edge, fwd.size), 4096, replace=False))])
+    bidx = np.sort(rs.choice(bwd.size, 8192, replace=False))
+    sums = lambda a: np.array([a.sum(dtype=np.float64), np.abs(a).sum(dtype=np.float64)])
+    out.update(roi_rois=rois, roi_fwd_idx=fidx.astype(np.int32), roi_fwd=fwd[fidx], roi_fwd_sums=sums(fwd),
+               roi_bwd_idx=bidx.astype(np.int32), roi_bwd=bwd[bidx], roi_bwd_sums=sums(bwd))
+    os.makedirs(out_dir, exist_ok=True)
+    np.savez_compressed(os.path.join(out_dir, "ref_kernels.npz"), **out)
+    print({k: v.shape for k, v in out.items()})
+
+
 def main():
     if len(sys.argv) > 1 and sys.argv[1] == "demo":
         return demo_goldens()
     if len(sys.argv) > 1 and sys.argv[1] == "solver":
         return solver_goldens()
+    if len(sys.argv) > 1 and sys.argv[1] == "ref_kernels":
+        return ref_kernel_goldens(*sys.argv[2:3])
     ref = ref_shim.load()
     cfg = ref.cfg
     calib = ref_shim.demo_calib()

@@ -1,7 +1,6 @@
 """GPU parity tests: hand-written sm_100a operators (through the C ABI) vs the CPU oracle, the
-committed goldens, and -- when oracle/_ref/libref_ops.so travelled with the snapshot -- the
-reference's own CUDA kernels compiled unmodified."""
-import ctypes
+committed goldens, and the outputs of the reference's own CUDA kernels compiled unmodified
+(tests/golden/ref_kernels.npz, minted by `make_golden.py ref_kernels`)."""
 import os
 
 import numpy as np
@@ -13,8 +12,6 @@ from stereo_rcnn_b200 import ops as G
 from stereo_rcnn_b200.synth import DEMO_P2, DEMO_P3, gen_rois, synth_pair
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SO = os.path.join(ROOT, "oracle", "_ref", "libref_ops.so")
 
 
 def cu(a):
@@ -34,10 +31,8 @@ def rand_dets(n, seed, size=600.0, wh=120.0):
 
 
 @pytest.fixture(scope="module")
-def reflib():
-    if not os.path.exists(REF_SO):
-        pytest.skip("oracle/_ref/libref_ops.so not present")
-    return ctypes.CDLL(REF_SO)
+def ref_kernels(golden_dir):
+    return np.load(os.path.join(golden_dir, "ref_kernels.npz"))
 
 
 # ------------------------------------------------------------------------ NMS
@@ -70,20 +65,16 @@ def test_nms_mask_upper_triangle_bits():
         assert not m[i, :i // 64].any() or cb == 1
 
 
-def test_nms_vs_reference_cuda_kernel(reflib):
-    """nms_cuda_compute of the reference (nms_cuda_kernel.cu:87-161), compiled unmodified"""
-    for n, seed in [(6000, 1), (1234, 2), (64, 3)]:
+NMS_REF_CASES = [(6000, 1), (1234, 2), (64, 3)]          # (boxes, seed of rand_dets), IoU 0.7
+
+
+def test_nms_vs_reference_cuda_kernel(ref_kernels):
+    """keep lists of nms_cuda_compute of the reference (nms_cuda_kernel.cu:87-161), compiled unmodified"""
+    for n, seed in NMS_REF_CASES:
         d = rand_dets(n, seed)
-        dd = cu(d)
-        keep = torch.zeros(n, dtype=torch.int32, device="cuda")
-        num = torch.zeros(1, dtype=torch.int32, device="cuda")
-        torch.cuda.synchronize()
-        reflib.nms_cuda_compute(ctypes.c_void_p(keep.data_ptr()), ctypes.c_void_p(num.data_ptr()),
-                                ctypes.c_void_p(dd.data_ptr()), n, 5, ctypes.c_float(0.7))
-        torch.cuda.synchronize()
-        ref_keep = keep[:int(num[0])].cpu().numpy()
+        ref_keep = ref_kernels["nms_keep_%d_%d" % (n, seed)]
         np.testing.assert_array_equal(ref_keep, O.nms(d, 0.7))              # pins the oracle
-        np.testing.assert_array_equal(G.nms(dd, 0.7).cpu().numpy().reshape(-1), ref_keep)
+        np.testing.assert_array_equal(G.nms(cu(d), 0.7).cpu().numpy().reshape(-1), ref_keep)
 
 
 # ------------------------------------------------------------------- RoIAlign
@@ -113,32 +104,49 @@ def test_roi_align_forward_vs_oracle(lat):
     assert (out.cpu().numpy() == ref).mean() > 0.999
 
 
-def test_roi_align_vs_reference_cuda_kernel(reflib):
+def roi_align_ref_inputs():
+    """feature map [1,32,40,60], 50 RoIs at spatial scale 0.25 and the top gradient [50,32,8,8] of the comparison with
+    the reference's RoIAlign kernels"""
     rs = np.random.RandomState(5)
     feat = rs.randn(1, 32, 40, 60).astype(np.float32)
     rois = rand_rois(50, 40, 60, 0.25, 2)
+    top = rs.randn(50, 32, 8, 8).astype(np.float32)
+    return feat, rois, top
+
+
+def test_roi_align_vs_reference_cuda_kernel(ref_kernels):
+    """ROIAlignForwardLaucher / ROIAlignBackwardLaucher of the reference (roi_align_kernel.cu), compiled unmodified.
+    The golden holds their outputs at a fixed sample of positions (every output of the two edge-case RoIs 0 and 1
+    included) and their sums over the whole output; ours and the oracle's full outputs are compared to each other."""
+    g = ref_kernels
+    feat, rois, top = roi_align_ref_inputs()
+    np.testing.assert_array_equal(rois, g["roi_rois"])
     f, r = cu(feat), cu(rois)
-    out_ref = torch.zeros(50, 32, 8, 8, device="cuda")
-    torch.cuda.synchronize()
-    reflib.ROIAlignForwardLaucher(ctypes.c_void_p(f.data_ptr()), ctypes.c_float(0.25), 50, 40, 60, 32, 8, 8,
-                                  ctypes.c_void_p(r.data_ptr()), ctypes.c_void_p(out_ref.data_ptr()),
-                                  ctypes.c_void_p(0))
-    torch.cuda.synchronize()
-    ref = out_ref.cpu().numpy()
-    np.testing.assert_allclose(O.roi_align_forward(feat, rois, 8, 8, np.float32(0.25)), ref, rtol=1e-6, atol=1e-6)
-    out = torch.zeros_like(out_ref)
+    out = torch.zeros(50, 32, 8, 8, device="cuda")
     G.roi_align_forward(8, 8, 0.25, f, r, out)
-    np.testing.assert_allclose(out.cpu().numpy(), ref, rtol=1e-6, atol=1e-6)
+    out = out.cpu().numpy()
+    ora = O.roi_align_forward(feat, rois, 8, 8, np.float32(0.25))
+    idx, ref = g["roi_fwd_idx"], g["roi_fwd"]
+    np.testing.assert_allclose(ora.reshape(-1)[idx], ref, rtol=1e-6, atol=1e-6)
+    np.testing.assert_allclose(out.reshape(-1)[idx], ref, rtol=1e-6, atol=1e-6)
+    np.testing.assert_allclose(out, ora, rtol=1e-6, atol=1e-6)
+    _check_sums(out, g["roi_fwd_sums"], 1e-6)
     # backward
-    top = cu(rs.randn(50, 32, 8, 8).astype(np.float32))
-    g_ref = torch.zeros(1, 32, 40, 60, device="cuda")
-    reflib.ROIAlignBackwardLaucher(ctypes.c_void_p(top.data_ptr()), ctypes.c_float(0.25), 1, 50, 40, 60, 32, 8, 8,
-                                   ctypes.c_void_p(r.data_ptr()), ctypes.c_void_p(g_ref.data_ptr()),
-                                   ctypes.c_void_p(0))
-    torch.cuda.synchronize()
-    g = torch.zeros_like(g_ref)
-    G.roi_align_backward(8, 8, 0.25, top, r, g)
-    np.testing.assert_allclose(g.cpu().numpy(), g_ref.cpu().numpy(), rtol=1e-4, atol=1e-4)
+    gr = torch.zeros(1, 32, 40, 60, device="cuda")
+    G.roi_align_backward(8, 8, 0.25, cu(top), r, gr)
+    gr = gr.cpu().numpy()
+    idx, ref = g["roi_bwd_idx"], g["roi_bwd"]
+    np.testing.assert_allclose(gr.reshape(-1)[idx], ref, rtol=1e-4, atol=1e-4)
+    np.testing.assert_allclose(gr, O.roi_align_backward(top, rois, feat.shape, 8, 8, np.float32(0.25)),
+                               rtol=1e-4, atol=1e-4)
+    _check_sums(gr, g["roi_bwd_sums"], 1e-4)
+
+
+def _check_sums(a, ref_sums, tol):
+    """(sum, sum of magnitudes) of `a` against the reference's: the bound elementwise |a - ref| <= tol + tol * |ref|
+    implies for both sums"""
+    got = [a.sum(dtype=np.float64), np.abs(a).sum(dtype=np.float64)]
+    np.testing.assert_allclose(got, ref_sums, rtol=0, atol=tol * (a.size + ref_sums[1]))
 
 
 def test_roi_align_backward_vs_oracle_and_autograd_module():

@@ -371,7 +371,7 @@ def test_record_gather_and_shard_equivalence_on_hardware(mode):
     N-GPU result equals the 1-GPU result on the same pairs"""
     world = min(torch.cuda.device_count(), 4)
     if world < 2:
-        pytest.skip("needs >= 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
