@@ -81,6 +81,20 @@ int sb_roi_align_pyramid_nhwc(const float* const* feats, const int* heights, con
                               int C, float im_h, const float* rois, int R, int pooled,
                               float* out, int out_ld, int out_coff, int round_tf32, sb_stream_t stream);
 
+/* Exact adjoint of sb_roi_align_pyramid_nhwc (PyramidRoI_Feat, stereo_rcnn.py:110-139, whose backward is the
+ * RoIAlignAvg autograd of modules/roi_align.py:26-29 -> roi_align_kernel.cu:94-143 per level): the same level routing,
+ * per-level scale, (P+1)^2 lattice and 2x2 average, transposed.  top_grad[r][ph][pw][top_coff + c] (row pitch top_ld)
+ * -> grad_feats[l] = N x H_l x W_l x C fp32, l = P2..P5, OVERWRITTEN.  Accumulated in 64-bit fixed point as
+ * sb_roi_align_backward_det (quantum max|top_grad| * 2^-41, found on the device): the result does not depend on the
+ * order of the atomics or of the RoIs -- bit-identical run to run.  C % 4 == 0.  A RoI whose batch index (column 0)
+ * is outside [0, N) contributes nothing (the forward reads such a RoI's taps unchecked; the backward never writes
+ * outside the feature gradients).                                                                                  */
+size_t sb_roi_align_pyramid_nhwc_backward_workspace(int N, const int* heights, const int* widths, int C);
+int sb_roi_align_pyramid_nhwc_backward(const float* top_grad, int top_ld, int top_coff, int C, float im_h,
+                                       const float* rois, int R, int pooled, int N, const int* heights,
+                                       const int* widths, float* const* grad_feats, void* workspace,
+                                       size_t workspace_bytes, sb_stream_t stream);
+
 /* ----------------------------------------------------- proposal layer ----
  * cls_prob [B,A,2] (column 1 = score), bbox_pred_lr [B,A,6], im_info [B,3] (device).
  * cfg: host struct (anchor pyramid + top-N / threshold constants), A = n_ratios*sum(h*w).
@@ -167,6 +181,28 @@ size_t sb_conv_trace_bytes(int max_launches);
 int sb_conv_trace(void* buf, int max_launches);
 int sb_conv_trace_count(void);
 int sb_conv_trace_info(int id, int* out12);
+
+/* GEMM on the tcgen05 tensor cores with operands read in their stored layout (the building block of the backward
+ * passes: weight gradients contract over pixels / RoIs, data gradients multiply by the untransposed weight -- the
+ * adjoints of the nn.Linear / 1x1 Conv2d products of resnet.py:256-263,282-285):
+ *   C[m][n] = alpha * sum_k A(m,k) * B(n,k) + bias[n]
+ * a, b: __half; a_mn_major = 0: A stored [M][lda], A(m,k) = a[m*lda + k];  1: stored [K][lda], A(m,k) = a[k*lda + m].
+ *       b_mn_major = 0: B stored [N][ldb];  1: stored [K][ldb], B(n,k) = b[k*ldb + n].
+ * c: fp32 [M][ldc] (overwritten).  alpha: DEVICE scalar or NULL (= 1), so that a scale computed on the device needs no
+ * host read (graph capturable).  bias: fp32 [N] or NULL.  fp32 accumulation; any M, N, K >= 1; lda / ldb / ldc
+ * multiples of 8 elements, a / b / c / bias 16-byte aligned (SB_EINVAL otherwise).  No split-K: C is bit-identical
+ * from run to run.  No transposed copy of an operand is made.                                                      */
+typedef struct {
+    const void* a;
+    const void* b;
+    float* c;
+    const float* alpha;
+    const float* bias;
+    int M, N, K;
+    int lda, ldb, ldc;
+    int a_mn_major, b_mn_major;
+} sb_gemm_desc;
+int sb_gemm_tc(const sb_gemm_desc* d, sb_stream_t stream);
 
 /* stem: NCHW image -> conv7x7/2 + frozen BN + ReLU -> NHWC (resnet.py:111-113) */
 int sb_stem_conv(const float* im_nchw, int N, int H, int W, const float* wgt /*[64][7][7][3]*/,
@@ -352,6 +388,32 @@ int sb_rcnn_loss(const float* cls_score, const float* bbox_pred, const float* di
                  float* d_right_border_pred, sb_stream_t stream);
 int sb_multitask_loss(const float* losses, const float* uncert, int n, float* total, float* d_uncert,
                       sb_stream_t stream);
+/* ------------------------------------------------- box-head training step (RCNN_top + tail, resnet.py:256-263,
+ * 282-285,345-348; stereo_rcnn.py:248-257).  The fc6 / fc7 products and their adjoints run through sb_gemm_tc.
+ * sb_dropout -- nn.Dropout(p = 0.2) after a ReLU with explicit random words (one uint32 per element, as the samplers
+ *   above): out = x * 1.25 where words[i] >= 0.2 * 2^32, else 0; out32 and / or out16 (__half).
+ * sb_box_tail_logits -- sb_box_tail writing the class LOGITS (the cross entropy of sb_rcnn_loss takes logits).
+ * sb_box_tail_backward -- adjoint of the three tail linears: d_fc7 [R,K] = [d_cls|d_bbox|d_dim] [Wc;Wb;Wd], and the
+ *   weight / bias gradients in the reference's shapes, fixed-order sums over R.
+ * sb_dropout_backward -- g = dy * keep * 1.25 * (y > 0) (y = the ReLU output the dropout consumed), db [C] = sum_r g
+ *   (fixed order; NULL: skipped), g16 = __half(g * 2^e) with e from max|g| on the device (largest element in
+ *   [2^14, 2^15)), inv_scale [1] = 2^-e for sb_gemm_tc's alpha.  No host read.
+ * sb_permute_pc_to_cp -- [Co][P][C] -> [Co][C][P] (the fc6 weight gradient from the GEMM's packed (ph, pw, c) order
+ *   to Conv2d's [2048][512][7][7]).                                                                                */
+int sb_dropout(const float* x, const unsigned* words, int R, int C, float* out32, void* out16, sb_stream_t stream);
+int sb_box_tail_logits(const float* fc7, int R, int K, int n_classes,
+                       const float* w_cls, const float* b_cls, const float* w_box, const float* b_box,
+                       const float* w_dim, const float* b_dim,
+                       float* cls_score, float* bbox_pred, float* dim_orien, sb_stream_t stream);
+int sb_box_tail_backward(const float* d_cls, const float* d_bbox, const float* d_dim, const float* fc7, int R, int K,
+                         int n_classes, const float* w_cls, const float* w_box, const float* w_dim, float* d_fc7,
+                         float* dw_cls, float* db_cls, float* dw_box, float* db_box, float* dw_dim, float* db_dim,
+                         sb_stream_t stream);
+size_t sb_dropout_backward_workspace(int R, int C);
+int sb_dropout_backward(const float* dy, const float* y, const unsigned* words, int R, int C, float* db, void* g16,
+                        float* inv_scale, void* workspace, size_t workspace_bytes, sb_stream_t stream);
+int sb_permute_pc_to_cp(const float* in, int Co, int P, int C, float* out, sb_stream_t stream);
+
 size_t sb_clip_gradient_workspace(int n_tensors);
 int sb_clip_gradient(float* const* grads, const size_t* counts, int n_tensors, float clip_norm,
                      void* workspace, size_t workspace_bytes, float* norm_out, sb_stream_t stream);

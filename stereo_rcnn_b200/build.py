@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libstereo_b200.so")
 SOURCES = ["misc.cu", "nms.cu", "proposal.cu", "roi_align.cu", "dense_align.cu", "conv_simt.cu", "conv_tc.cu", "peer.cu", "box_solver.cu",
-           "train_targets.cu", "train_loss.cu"]
+           "train_targets.cu", "train_loss.cu", "train_backward.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",
          "-Xcompiler", "-Wall", "-Xcompiler", "-Wno-unused-function"]

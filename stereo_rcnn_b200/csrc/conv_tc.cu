@@ -616,27 +616,41 @@ struct FlatParams {
     // STEM variant: the A operand is gathered from the NCHW fp32 image (7x7 / stride 2 / pad 3 patches), no im2col
     const float* stem_im;
     int sH, sW, sHo, sWo;
+    // GEMM variant (sb_gemm_tc): out = alpha * acc + shift[col], alpha read from device memory (NULL: 1)
+    const float* alpha;
 };
 
-constexpr int flat_epi_warp_bytes(bool res, bool f32) { return f32 ? ((res ? 3 : 2) * 4096 + 4096) : 4096; }
+// per epilogue warp: NB fp32 boxes + the fp16 twin's two half boxes (the GEMM variant stores no twin)
+constexpr int flat_epi_warp_bytes(bool res, bool f32, bool gemm = false) {
+    return f32 ? ((res ? 3 : 2) * 4096 + (gemm ? 0 : 4096)) : 4096;
+}
 
 constexpr int kStemGatherWarps = 8;       // 2 threads per A-tile row: each builds 4 of the 8 16-byte groups of a K-step
 constexpr int kStemThreads = 320 + 32 * kStemGatherWarps;
 
-template <int BLOCK_N, int kStages, bool HAS_RES, bool F32, bool STEM = false>
+// GEMM variant (sb_gemm_tc, C = alpha * A B^T + bias): A_MN / B_MN select an operand stored M/N-major ([K][ld]).  Its
+// tiles arrive as 64-element-wide TMA boxes (the 128-byte swizzle span) of BLOCK_K K rows each -- 2 for A, BLOCK_N / 64
+// for B, stacked 8 KB apart -- and the MMAs read them through M/N-major descriptors with the transpose bits set, so no
+// transposed copy of an operand ever exists.  Everything else (pipeline, TMEM double buffer, TMA-store epilogue) is
+// the conv's.
+template <int BLOCK_N, int kStages, bool HAS_RES, bool F32, bool STEM = false, bool GEMM = false, bool A_MN = false,
+          bool B_MN = false>
 __global__ void __launch_bounds__(STEM ? kStemThreads : 320, 1)
 conv_tc_flat_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                     const __grid_constant__ CUtensorMap map_res, const __grid_constant__ CUtensorMap map_o32,
                     const __grid_constant__ CUtensorMap map_o16, const FlatParams p) {
     static_assert(!HAS_RES || F32, "the residual epilogue produces the fp32 stream");
+    static_assert(GEMM || (!A_MN && !B_MN), "M/N-major operands are a GEMM feature");
+    static_assert(!B_MN || BLOCK_N % 64 == 0, "M/N-major B tiles are whole 64-element boxes");
+    constexpr uint32_t kMnBox = 64 * 64 * 2;      // one M/N-major TMA box: 64 M/N elements x 64 K rows of fp16
     constexpr uint32_t kABytes = BLOCK_M * kRowBytes, kBBytes = BLOCK_N * kRowBytes;
     constexpr int BLOCK_K = 64;
     constexpr uint32_t kStageBytes = kABytes + kBBytes;
     constexpr uint32_t kTmemCols = (2 * BLOCK_N <= 32) ? 32 : (2 * BLOCK_N <= 64) ? 64 : (2 * BLOCK_N <= 128) ? 128
                                    : (2 * BLOCK_N <= 256) ? 256 : 512;
     constexpr int NB = HAS_RES ? 3 : 2;                                  // fp32 boxes per warp
-    constexpr int kEpiWarpBytes = flat_epi_warp_bytes(HAS_RES, F32);
-    constexpr int kF16Off = F32 ? NB * 4096 : 0;
+    constexpr int kEpiWarpBytes = flat_epi_warp_bytes(HAS_RES, F32, GEMM);
+    constexpr int kF16Off = F32 ? NB * 4096 : 0;       // (GEMM: no twin, has16 = 0)
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     uint8_t* epi = smem + kStages * kStageBytes;                          // 1024-aligned (stage bytes are multiples of 4096)
@@ -696,15 +710,29 @@ conv_tc_flat_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                     mbar_wait(&empty[stage], phase ^ 1);
                     uint8_t* sa = smem + stage * kStageBytes;
                     mbar_expect_tx(&full[stage], STEM ? kBBytes : kStageBytes);
-                    if (!STEM) tma_load_2d(&map_a, &full[stage], sa, kb * BLOCK_K, mt * BLOCK_M);
-                    tma_load_2d(&map_b, &full[stage], sa + kABytes, kb * BLOCK_K, nt * BLOCK_N);
+                    if (A_MN) {
+#pragma unroll
+                        for (int i = 0; i < BLOCK_M / 64; ++i)
+                            tma_load_2d(&map_a, &full[stage], sa + i * kMnBox, mt * BLOCK_M + 64 * i, kb * BLOCK_K);
+                    } else if (!STEM) {
+                        tma_load_2d(&map_a, &full[stage], sa, kb * BLOCK_K, mt * BLOCK_M);
+                    }
+                    if (B_MN) {
+#pragma unroll
+                        for (int i = 0; i < BLOCK_N / 64; ++i)
+                            tma_load_2d(&map_b, &full[stage], sa + kABytes + i * kMnBox, nt * BLOCK_N + 64 * i, kb * BLOCK_K);
+                    } else {
+                        tma_load_2d(&map_b, &full[stage], sa + kABytes, kb * BLOCK_K, nt * BLOCK_N);
+                    }
                     if (++stage == kStages) { stage = 0; phase ^= 1; }
                 }
             }
         }
     } else if (warp == 1) {
         // ===================== MMA issuer =====================
-        constexpr uint32_t idesc = make_idesc(BLOCK_N, true);
+        constexpr uint32_t idesc = make_idesc_major(BLOCK_N, true, A_MN, B_MN);
+        // per MMA (K = 16): K-major operands advance 32 bytes inside the swizzle row, M/N-major ones two 8-row K groups
+        constexpr uint64_t kStepA = A_MN ? 2048 >> 4 : 2, kStepB = B_MN ? 2048 >> 4 : 2;
         int stage = 0;
         uint32_t phase = 0;
         int acc = 0;
@@ -719,10 +747,11 @@ conv_tc_flat_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                 if (tr && lane == 0 && kb == 0 && tile == (int)blockIdx.x) { tr[2] = gtimer(); tr[10] = clock64(); }
                 if (elect_one()) {
                     const uint32_t sa = smem_u32(smem + stage * kStageBytes);
-                    const uint64_t da = make_smem_desc(sa), db = make_smem_desc(sa + kABytes);
+                    const uint64_t da = A_MN ? make_smem_desc_mn(sa, kMnBox) : make_smem_desc(sa);
+                    const uint64_t db = B_MN ? make_smem_desc_mn(sa + kABytes, kMnBox) : make_smem_desc(sa + kABytes);
 #pragma unroll
                     for (int k = 0; k < 4; ++k)
-                        umma_f16(tmem_d, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc, (kb | k) != 0);
+                        umma_f16(tmem_d, da + (uint64_t)k * kStepA, db + (uint64_t)k * kStepB, idesc, (kb | k) != 0);
                     umma_commit(&empty[stage]);
                     if (kb == p.num_k_blocks - 1) umma_commit(&tfull[acc]);
                 }
@@ -824,6 +853,8 @@ conv_tc_flat_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         uint64_t* my_rfull = rfull + ew * 3;
         const bool has16 = p.has16 != 0;
         const bool relu = p.relu != 0;
+        // (after griddepcontrol.wait: alpha may come from the kernel just before)
+        const float alpha = (GEMM && p.alpha) ? __ldg(p.alpha) : 1.f;
         uint32_t g = 0;                    // running chunk number of this warp (ring position)
         // coordinates of chunk gi in this warp's chunk sequence (tiles of this CTA x chunks of the warp)
         auto issue_res = [&](uint32_t gi) {
@@ -880,8 +911,21 @@ conv_tc_flat_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                     for (int j = 0; j < 8; ++j) {
                         const int cj = c0 + 4 * j;
                         const bool ok = cj < p.Cout;
-                        const float4 sc = (p.scale && ok) ? __ldg(reinterpret_cast<const float4*>(p.scale + cj)) : make_float4(1.f, 1.f, 1.f, 1.f);
-                        const float4 sh = (p.shift && ok) ? __ldg(reinterpret_cast<const float4*>(p.shift + cj)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                        float4 sc, sh;
+                        if (GEMM) {      // any N: the bias of a partial column quad is read element by element
+                            sc = make_float4(alpha, alpha, alpha, alpha);
+                            sh = make_float4(0.f, 0.f, 0.f, 0.f);
+                            if (p.shift && cj + 4 <= p.Cout) {
+                                sh = __ldg(reinterpret_cast<const float4*>(p.shift + cj));
+                            } else if (p.shift && ok) {
+                                sh.x = __ldg(p.shift + cj);
+                                if (cj + 1 < p.Cout) sh.y = __ldg(p.shift + cj + 1);
+                                if (cj + 2 < p.Cout) sh.z = __ldg(p.shift + cj + 2);
+                            }
+                        } else {
+                            sc = (p.scale && ok) ? __ldg(reinterpret_cast<const float4*>(p.scale + cj)) : make_float4(1.f, 1.f, 1.f, 1.f);
+                            sh = (p.shift && ok) ? __ldg(reinterpret_cast<const float4*>(p.shift + cj)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                        }
                         float4 x;
                         x.x = fmaf(__uint_as_float(v[4 * j + 0]), sc.x, sh.x);
                         x.y = fmaf(__uint_as_float(v[4 * j + 1]), sc.y, sh.y);
@@ -1070,16 +1114,16 @@ int launch(const CUtensorMap& ma, const CUtensorMap& mb, const TcParams& p, cuda
 }
 
 
-template <int BN, int ST, bool RES, bool F32, bool STEM = false>
+template <int BN, int ST, bool RES, bool F32, bool STEM = false, bool GEMM = false, bool A_MN = false, bool B_MN = false>
 int launch_flat(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mr, const CUtensorMap& mo32,
                 const CUtensorMap& mo16, const FlatParams& p, int max_ctas, cudaStream_t st) {
-    constexpr size_t smem = (size_t)ST * (BLOCK_M * kRowBytes + BN * kRowBytes) + 8 * (size_t)flat_epi_warp_bytes(RES, F32) +
+    constexpr size_t smem = (size_t)ST * (BLOCK_M * kRowBytes + BN * kRowBytes) + 8 * (size_t)flat_epi_warp_bytes(RES, F32, GEMM) +
                             (2 * ST + 4 + 24) * 8 + 16 + 1024;
     static_assert(smem <= 227 * 1024, "smem budget");
     static bool attr_done[kSbMaxDevices] = {false};
     bool& attr = attr_done[sb_cur_device()];
     if (!attr) {
-        cudaError_t e = cudaFuncSetAttribute(conv_tc_flat_kernel<BN, ST, RES, F32, STEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(conv_tc_flat_kernel<BN, ST, RES, F32, STEM, GEMM, A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
         attr = true;
     }
@@ -1098,7 +1142,7 @@ int launch_flat(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap&
     attrs[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attrs;
     cfg.numAttrs = use_pdl ? 1 : 0;
-    cudaError_t le = cudaLaunchKernelEx(&cfg, conv_tc_flat_kernel<BN, ST, RES, F32, STEM>, ma, mb, mr, mo32, mo16, p);
+    cudaError_t le = cudaLaunchKernelEx(&cfg, conv_tc_flat_kernel<BN, ST, RES, F32, STEM, GEMM, A_MN, B_MN>, ma, mb, mr, mo32, mo16, p);
     SB_LAUNCHED();
     if (le != cudaSuccess) return (int)le;
     SB_CHECK_LAUNCH();
@@ -1261,6 +1305,7 @@ extern "C" int sb_conv2d_tc(const sb_conv_desc* d, sb_stream_t stream) {
         fp.num_m_tiles = p.num_m_tiles; fp.num_n_tiles = p.num_n_tiles; fp.num_k_blocks = p.num_k_blocks;
         fp.relu = d->relu; fp.has16 = d->out16 ? 1 : 0; fp.pdl_late = p.pdl_late; fp.trace = p.trace;
         fp.stem_im = nullptr; fp.sH = fp.sW = fp.sHo = fp.sWo = 0;
+        fp.alpha = nullptr;
         CUtensorMap mr = ma, mo32 = ma, mo16 = ma;      // unused maps still need a valid descriptor
         const cuuint64_t dims[2] = {(cuuint64_t)d->Cout, (cuuint64_t)p.M};
         const cuuint32_t box[2] = {32, 32};
@@ -1322,6 +1367,7 @@ extern "C" int sb_stem_conv_tc(const float* im_nchw, int N, int H, int W, const 
     fp.pdl_late = pdl_late ? 1 : 0;
     fp.trace = nullptr;
     fp.stem_im = im_nchw; fp.sH = H; fp.sW = W; fp.sHo = Ho; fp.sWo = Wo;
+    fp.alpha = nullptr;
     CUtensorMap mb, mo16;
     {
         cuuint64_t dims[2] = {192, 64};
@@ -1336,4 +1382,71 @@ extern "C" int sb_stem_conv_tc(const float* im_nchw, int N, int H, int W, const 
         if (!make_map(&mo16, out16, 2, dims, str, box, true, CU_TENSOR_MAP_SWIZZLE_64B)) return SB_EINVAL;
     }
     return launch_flat<64, 8, false, false, true>(mb, mb, mb, mb, mo16, fp, 0, sb_cs(stream));
+}
+
+// ------------------------------------------------------------------ GEMM with transposed operands
+// C[m][n] = alpha * sum_k A(m,k) B(n,k) + bias[n] through the flat kernel's pipeline (conv_tc_flat_kernel<.., GEMM>):
+// 128 x 256 tiles (3 stages of 48 KB) or 128 x 128 (4 stages of 32 KB), fp32 C leaves through 32 x 32 TMA boxes.  The backward passes of the layers need
+// the operands in the layout their forward stored them in: weight gradients contract over pixels / RoIs (both
+// operands M/N-major), data gradients multiply by the untransposed weight (B N-major).  Tails in M, N and K are
+// zero-filled by the load maps and clipped by the store map.  One CTA owns each output tile and walks K in order (no
+// split-K), so C is bit-identical from run to run.
+namespace {
+// 256-wide tiles: 3 stages of 48 KB beside the 64 KB of fp32 boxes (the GEMM stores no fp16 twin)
+template <bool A_MN, bool B_MN>
+int launch_gemm(int bn, const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mo32, const FlatParams& fp,
+                cudaStream_t st) {
+    if (bn == 256) return launch_flat<256, 3, false, true, false, true, A_MN, B_MN>(ma, mb, mo32, mo32, mo32, fp, 0, st);
+    return launch_flat<128, 4, false, true, false, true, A_MN, B_MN>(ma, mb, mo32, mo32, mo32, fp, 0, st);
+}
+}  // namespace
+
+extern "C" int sb_gemm_tc(const sb_gemm_desc* d, sb_stream_t stream) {
+    if (!d || !d->a || !d->b || !d->c || d->M < 1 || d->N < 1 || d->K < 1) return SB_EINVAL;
+    if ((d->lda & 7) || (d->ldb & 7) || (d->ldc & 7)) return SB_EINVAL;
+    if (d->lda < (d->a_mn_major ? d->M : d->K) || d->ldb < (d->b_mn_major ? d->N : d->K) || d->ldc < d->N) return SB_EINVAL;
+    if ((reinterpret_cast<uintptr_t>(d->a) & 15) || (reinterpret_cast<uintptr_t>(d->b) & 15) ||
+        (reinterpret_cast<uintptr_t>(d->c) & 15) || (reinterpret_cast<uintptr_t>(d->bias) & 15) ||
+        (reinterpret_cast<uintptr_t>(d->alpha) & 3))
+        return SB_EINVAL;
+    const long long m_tiles = ((long long)d->M + BLOCK_M - 1) / BLOCK_M;
+    if (m_tiles >= 0x7fffffffLL) return SB_EINVAL;
+    // 256-wide tiles carry 48 KB per 512 MMA cycles instead of 32 KB per 256: the wide tile is less bound by L2 bandwidth
+    // (pick_block_n's cost model, which also weighs the waves of the persistent grid)
+    const int BN = (d->N >= 256 && pick_block_n(d->N, m_tiles, sb_num_sms()) == 256) ? 256 : 128;
+    const long long n_tiles = ((long long)d->N + BN - 1) / BN;
+    if (m_tiles * n_tiles >= 0x7fffffffLL) return SB_EINVAL;
+    FlatParams fp;
+    fp.scale = nullptr; fp.shift = d->bias; fp.residual = nullptr;
+    fp.M = d->M; fp.Cout = d->N; fp.res_ld = 0;
+    fp.num_m_tiles = (int)m_tiles; fp.num_n_tiles = (int)n_tiles; fp.num_k_blocks = (d->K + 63) / 64;
+    fp.relu = 0; fp.has16 = 0;
+    static const bool pdl_late = getenv("SB_PDL_LATE") == nullptr || atoi(getenv("SB_PDL_LATE")) != 0;
+    fp.pdl_late = pdl_late ? 1 : 0;
+    fp.trace = nullptr;
+    fp.stem_im = nullptr; fp.sH = fp.sW = fp.sHo = fp.sWo = 0;
+    fp.alpha = d->alpha;
+    CUtensorMap ma, mb, mo;
+    {   // K-major: rows of K elements, box 64 (K) x 128 rows;  M-major: rows of M elements, box 64 (M) x 64 K rows
+        const cuuint64_t dims[2] = {(cuuint64_t)(d->a_mn_major ? d->M : d->K), (cuuint64_t)(d->a_mn_major ? d->K : d->M)};
+        const cuuint64_t str[1] = {(cuuint64_t)d->lda * 2};
+        const cuuint32_t box[2] = {64, d->a_mn_major ? 64u : (cuuint32_t)BLOCK_M};
+        if (!make_map(&ma, d->a, 2, dims, str, box, true)) return SB_EINVAL;
+    }
+    {
+        const cuuint64_t dims[2] = {(cuuint64_t)(d->b_mn_major ? d->N : d->K), (cuuint64_t)(d->b_mn_major ? d->K : d->N)};
+        const cuuint64_t str[1] = {(cuuint64_t)d->ldb * 2};
+        const cuuint32_t box[2] = {64, d->b_mn_major ? 64u : (cuuint32_t)BN};
+        if (!make_map(&mb, d->b, 2, dims, str, box, true)) return SB_EINVAL;
+    }
+    {
+        const cuuint64_t dims[2] = {(cuuint64_t)d->N, (cuuint64_t)d->M};
+        const cuuint64_t str[1] = {(cuuint64_t)d->ldc * 4};
+        const cuuint32_t box[2] = {32, 32};
+        if (!make_map(&mo, d->c, 2, dims, str, box, false)) return SB_EINVAL;
+    }
+    cudaStream_t st = sb_cs(stream);
+    if (d->a_mn_major)
+        return d->b_mn_major ? launch_gemm<true, true>(BN, ma, mb, mo, fp, st) : launch_gemm<true, false>(BN, ma, mb, mo, fp, st);
+    return d->b_mn_major ? launch_gemm<false, true>(BN, ma, mb, mo, fp, st) : launch_gemm<false, false>(BN, ma, mb, mo, fp, st);
 }

@@ -191,6 +191,9 @@ kpts_softmax_kernel(const float* __restrict__ pred_all, int G, float* __restrict
 }
 
 // box tail (stereo_rcnn.py:253-257): three linears on fc7 + softmax over classes
+// LOGITS = false: softmax probabilities (test time, sb_box_tail); true: the raw class scores (sb_box_tail_logits, the
+// training forward: the cross entropy of sb_rcnn_loss takes logits)
+template <bool LOGITS>
 __global__ void __launch_bounds__(256)
 box_tail_kernel(const float* __restrict__ fc7, int K, int nc, const float* __restrict__ w_cls,
                 const float* __restrict__ b_cls, const float* __restrict__ w_box,
@@ -218,7 +221,8 @@ box_tail_kernel(const float* __restrict__ fc7, int K, int nc, const float* __res
         outv[tid] = s;
     }
     __syncthreads();
-    if (tid == 0) {
+    if (LOGITS && tid < nc) cls_prob[(size_t)r * nc + tid] = outv[tid];
+    if (!LOGITS && tid == 0) {
         float m = -INFINITY, s = 0.f;
         for (int j = 0; j < nc; ++j) m = fmaxf(m, outv[j]);
         for (int j = 0; j < nc; ++j) s += expf(outv[j] - m);
@@ -484,8 +488,20 @@ extern "C" int sb_box_tail(const float* fc7, int R, int K, int n_classes, const 
                            float* cls_prob, float* bbox_pred, float* dim_orien, sb_stream_t stream) {
     if (R == 0) return SB_OK;
     if (n_classes < 1 || n_classes > 4) return SB_EINVAL;
-    box_tail_kernel<<<R, 256, 0, sb_cs(stream)>>>(fc7, K, n_classes, w_cls, b_cls, w_box, b_box, w_dim, b_dim,
-                                                  cls_prob, bbox_pred, dim_orien);
+    box_tail_kernel<false><<<R, 256, 0, sb_cs(stream)>>>(fc7, K, n_classes, w_cls, b_cls, w_box, b_box, w_dim, b_dim,
+                                                         cls_prob, bbox_pred, dim_orien);
+    SB_LAUNCHED();
+    SB_CHECK_LAUNCH();
+    return SB_OK;
+}
+
+extern "C" int sb_box_tail_logits(const float* fc7, int R, int K, int n_classes, const float* w_cls, const float* b_cls,
+                                  const float* w_box, const float* b_box, const float* w_dim, const float* b_dim,
+                                  float* cls_score, float* bbox_pred, float* dim_orien, sb_stream_t stream) {
+    if (R == 0) return SB_OK;
+    if (n_classes < 1 || n_classes > 4) return SB_EINVAL;
+    box_tail_kernel<true><<<R, 256, 0, sb_cs(stream)>>>(fc7, K, n_classes, w_cls, b_cls, w_box, b_box, w_dim, b_dim,
+                                                        cls_score, bbox_pred, dim_orien);
     SB_LAUNCHED();
     SB_CHECK_LAUNCH();
     return SB_OK;

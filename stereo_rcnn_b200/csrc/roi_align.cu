@@ -186,15 +186,25 @@ __device__ __forceinline__ int roi_level(const float* roi) {
     return (int)l - 2;
 }
 
+// the geometry of one lattice tap of a pyramid RoI on NHWC features (forward and backward share it)
+struct TapRec {
+    double w00, w01, w10, w11;
+    long long off;      // element offset of the top-left source pixel, or -1 for a zero tap
+};
+
+__device__ __forceinline__ TapRec tap_record(const RoiGeom& g, int ph, int pw, int H, int W, int C) {
+    const Tap t = make_tap(g, ph, pw, H, W);
+    TapRec tr;
+    tr.w00 = t.w00; tr.w01 = t.w01; tr.w10 = t.w10; tr.w11 = t.w11;
+    tr.off = t.zero ? -1 : (long long)((((size_t)g.batch * H + t.h0) * W + t.w0) * C);
+    return tr;
+}
+
 // One CTA per (roi, block of RB output rows); C % 4 == 0.  The CTA walks the RB+1 lattice rows of its block with a
 // rolling pair of rows in shared memory (each lattice row is built once per CTA instead of once per output row: at
 // RB = 7 the 14x14 pooling does 8/7 instead of 2x the tap work), and the tap geometry -- fp64 weights, offsets -- is
 // built once per (row, column) by the first threads instead of once per channel vector.
 // dynamic smem = 2 * (P+1) * C floats for the lattice rows + (RB+1) * (P+1) tap records.
-struct TapRec {
-    double w00, w01, w10, w11;
-    long long off;      // element offset of the top-left source pixel, or -1 for a zero tap
-};
 
 __global__ void __launch_bounds__(256)
 roi_align_pyramid_nhwc(PyramidArgs a, int C, const float* __restrict__ rois, int P, int RB,
@@ -213,11 +223,7 @@ roi_align_pyramid_nhwc(PyramidArgs a, int C, const float* __restrict__ rois, int
     const RoiGeom g = roi_geom(roi, a.scale[lv], L, L);
     for (int e = threadIdx.x; e < (rows + 1) * L; e += blockDim.x) {
         const int r = e / L, pw = e - r * L;
-        const Tap t = make_tap(g, ph0 + r, pw, H, W);
-        TapRec tr;
-        tr.w00 = t.w00; tr.w01 = t.w01; tr.w10 = t.w10; tr.w11 = t.w11;
-        tr.off = t.zero ? -1 : (long long)((((size_t)g.batch * H + t.h0) * W + t.w0) * C);
-        taps[e] = tr;
+        taps[e] = tap_record(g, ph0 + r, pw, H, W, C);
     }
     __syncthreads();
     const size_t wstep = (size_t)W * C4;
@@ -269,6 +275,72 @@ roi_align_pyramid_nhwc(PyramidArgs a, int C, const float* __restrict__ rois, int
         __syncthreads();       // the next lattice row overwrites `top`
     }
 }
+
+// ---- adjoint of roi_align_pyramid_nhwc, deterministic: the fixed-point scatter of roi_align_bwd_fixed_kernel on the
+// forward's routing and tap geometry.  Lattice point (i, j) feeds the output cells (i-1..i, j-1..j) of the 2x2 average
+// with weight 1/4 each, so its gradient is 1/4 of the sum of those cells' gradients (fp64, fixed order); it then goes
+// to the tap's four source pixels with the tap's fp64 weights.  One CTA per RoI; threads sweep (tap, channel) with the
+// channel fastest, so the 64-bit atomics of a warp hit consecutive words.
+struct PyramidGradArgs {
+    unsigned long long* acc[4];
+    int H[4], W[4];
+    float scale[4];
+};
+
+__global__ void __launch_bounds__(256)
+absmax_rows_kernel(const float* __restrict__ x, size_t rows, int cols, int ld, unsigned* __restrict__ out) {
+    unsigned m = 0u;
+    const size_t n = rows * (size_t)cols;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t r = i / (size_t)cols, c = i - r * (size_t)cols;
+        const unsigned b = __float_as_uint(x[r * (size_t)ld + c]) & 0x7fffffffu;
+        m = b > m ? b : m;
+    }
+    m = __reduce_max_sync(0xffffffffu, m);
+    if ((threadIdx.x & 31) == 0 && m) atomicMax(out, m);
+}
+
+__global__ void __launch_bounds__(256)
+roi_align_pyramid_nhwc_bwd_fixed(PyramidGradArgs a, int N, int C, const float* __restrict__ rois, int P,
+                                 const float* __restrict__ top, int top_ld, const unsigned* __restrict__ absmax) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    TapRec* taps = reinterpret_cast<TapRec*>(smem_raw);      // [L][L]
+    const int L = P + 1;
+    const int n = blockIdx.x;
+    const float* roi = rois + 5 * n;
+    const int lv = roi_level(roi);
+    const int H = a.H[lv], W = a.W[lv];
+    const RoiGeom g = roi_geom(roi, a.scale[lv], L, L);
+    if (g.batch < 0 || g.batch >= N) return;      // no image of the batch: nothing to scatter (whole CTA leaves)
+    for (int e = threadIdx.x; e < L * L; e += blockDim.x) taps[e] = tap_record(g, e / L, e % L, H, W, C);
+    __syncthreads();
+    const double s = ldexp(1.0, fixed_exponent(*absmax));
+    const float* __restrict__ tg = top + (size_t)n * P * P * top_ld;
+    unsigned long long* __restrict__ acc = a.acc[lv];
+    const size_t wstep = (size_t)W * C;
+    for (int e = threadIdx.x; e < L * L * C; e += blockDim.x) {
+        const int t = e / C, c = e - t * C;
+        const TapRec& tr = taps[t];
+        if (tr.off < 0) continue;
+        const int i = t / L, j = t - i * L;
+        double gs = 0.;
+        for (int oh = i - 1; oh <= i; ++oh) {
+            if (oh < 0 || oh >= P) continue;
+            if (j >= 1) gs += (double)tg[((size_t)oh * P + j - 1) * top_ld + c];
+            if (j < P) gs += (double)tg[((size_t)oh * P + j) * top_ld + c];
+        }
+        if (gs == 0.) continue;
+        const double tv = 0.25 * gs * s;
+        unsigned long long* b = acc + tr.off + c;
+        atomicAdd(b, (unsigned long long)__double2ll_rn(tv * tr.w00));       // two's complement: wraps like int64
+        atomicAdd(b + C, (unsigned long long)__double2ll_rn(tv * tr.w01));
+        atomicAdd(b + wstep, (unsigned long long)__double2ll_rn(tv * tr.w10));
+        atomicAdd(b + wstep + C, (unsigned long long)__double2ll_rn(tv * tr.w11));
+    }
+}
+
+// stereo_rcnn.py:128: scale = feat.size(2) / im_info[0][0] (python float), then float(...)
+float pyramid_scale(int height, float im_h) { return (float)((double)height / (double)im_h); }
 
 }  // namespace
 
@@ -340,8 +412,7 @@ extern "C" int sb_roi_align_pyramid_nhwc(const float* const* feats, const int* h
         a.feat[l] = feats[l];
         a.H[l] = heights[l];
         a.W[l] = widths[l];
-        // stereo_rcnn.py:128: scale = feat.size(2) / im_info[0][0] (python float), then float(...)
-        a.scale[l] = (float)((double)heights[l] / (double)im_h);
+        a.scale[l] = pyramid_scale(heights[l], im_h);
     }
     // output rows per CTA: all of a 7x7 tile (8 lattice rows for 7 outputs), half of a 14x14 tile
     int RB = pooled <= 8 ? pooled : (pooled + 1) / 2;
@@ -359,6 +430,63 @@ extern "C" int sb_roi_align_pyramid_nhwc(const float* const* feats, const int* h
     dim3 grid(R, (pooled + RB - 1) / RB);
     roi_align_pyramid_nhwc<<<grid, 256, smem, sb_cs(stream)>>>(a, C, rois, pooled, RB, out, out_ld, out_coff, round_tf32);
     SB_LAUNCHED();
+    SB_CHECK_LAUNCH();
+    return SB_OK;
+}
+
+extern "C" size_t sb_roi_align_pyramid_nhwc_backward_workspace(int N, const int* heights, const int* widths, int C) {
+    if (N < 1 || C < 1 || !heights || !widths) return 0;
+    size_t n = 0;
+    for (int l = 0; l < 4; ++l) {
+        if (heights[l] < 2 || widths[l] < 2) return 0;
+        n += (size_t)N * heights[l] * widths[l] * C;
+    }
+    return n * 8 + 16;
+}
+
+extern "C" int sb_roi_align_pyramid_nhwc_backward(const float* top_grad, int top_ld, int top_coff, int C, float im_h,
+                                                  const float* rois, int R, int pooled, int N, const int* heights,
+                                                  const int* widths, float* const* grad_feats, void* workspace,
+                                                  size_t workspace_bytes, sb_stream_t stream) {
+    if (R < 0 || C < 4 || (C & 3) || pooled < 1 || N < 1 || top_coff < 0 || top_ld < top_coff + C || !heights ||
+        !widths || !grad_feats || (R > 0 && (!top_grad || !rois)) || !workspace || (reinterpret_cast<uintptr_t>(workspace) & 7))
+        return SB_EINVAL;
+    const size_t need = sb_roi_align_pyramid_nhwc_backward_workspace(N, heights, widths, C);
+    if (need == 0 || workspace_bytes < need) return SB_EINVAL;
+    for (int l = 0; l < 4; ++l)
+        if (!grad_feats[l]) return SB_EINVAL;
+    const int L = pooled + 1;
+    const size_t smem = (size_t)L * L * sizeof(TapRec);
+    if (smem > 48 * 1024) return SB_EINVAL;
+    PyramidGradArgs a;
+    size_t cnt[4], off = 0;
+    unsigned long long* acc = static_cast<unsigned long long*>(workspace);
+    for (int l = 0; l < 4; ++l) {
+        cnt[l] = (size_t)N * heights[l] * widths[l] * C;
+        a.acc[l] = acc + off;
+        off += cnt[l];
+        a.H[l] = heights[l];
+        a.W[l] = widths[l];
+        a.scale[l] = pyramid_scale(heights[l], im_h);
+    }
+    unsigned* absmax = reinterpret_cast<unsigned*>(acc + off);
+    cudaStream_t st = sb_cs(stream);
+    cudaError_t e = cudaMemsetAsync(workspace, 0, need, st);
+    if (e != cudaSuccess) return (int)e;
+    if (R > 0) {
+        const size_t rows = (size_t)R * pooled * pooled, nt = rows * C;
+        absmax_rows_kernel<<<(int)((nt + 255) / 256 < 1184 ? (nt + 255) / 256 : 1184), 256, 0, st>>>(
+            top_grad + top_coff, rows, C, top_ld, absmax);
+        SB_LAUNCHED();
+        roi_align_pyramid_nhwc_bwd_fixed<<<R, 256, smem, st>>>(a, N, C, rois, pooled, top_grad + top_coff, top_ld, absmax);
+        SB_LAUNCHED();
+    }
+    for (int l = 0; l < 4; ++l) {
+        const size_t n = cnt[l];
+        fixed_to_float_kernel<<<(int)((n + 255) / 256 < 2368 ? (n + 255) / 256 : 2368), 256, 0, st>>>(a.acc[l], n, absmax,
+                                                                                                     grad_feats[l]);
+        SB_LAUNCHED();
+    }
     SB_CHECK_LAUNCH();
     return SB_OK;
 }

@@ -71,11 +71,29 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
     return d;
 }
 
+// M/N-major, 128-byte swizzle descriptor (the operand is stored with M or N contiguous): one swizzle atom is 64 M/N
+// elements (one 128-byte row) x 8 K rows (1024 B).  Here SBO is the step between 8-row K groups (1024 B: the K rows of
+// a TMA box follow each other) and LBO the step between 64-element M/N blocks (`mn_block_bytes`: one TMA box each).
+// An MMA with K = 16 reads two K groups; the next one starts 2048 B further on.
+__device__ __forceinline__ uint64_t make_smem_desc_mn(uint32_t saddr, uint32_t mn_block_bytes) {
+    uint64_t d = 0;
+    d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
+    d |= (uint64_t)(mn_block_bytes >> 4) << 16;
+    d |= (uint64_t)(1024 >> 4) << 32;
+    d |= (uint64_t)1 << 46;
+    d |= (uint64_t)2 << 61;
+    return d;
+}
+
 // kind::tf32 instruction descriptor (cute::UMMA::InstrDescriptor): D=F32 (1<<4), A=TF32 (2<<7),
 // B=TF32 (2<<10), A/B K-major (bits 15/16 = 0), N>>3 at [17,23), M>>4 at [24,29)
 __host__ __device__ constexpr uint32_t make_idesc(int n, bool f16) {
     return (1u << 4) | ((f16 ? 0u : 2u) << 7) | ((f16 ? 0u : 2u) << 10) | ((uint32_t)(n >> 3) << 17) |
            ((uint32_t)(BLOCK_M >> 4) << 24);
+}
+// the same with the transpose bits: A (bit 15) and / or B (bit 16) read M/N-major from shared memory
+__host__ __device__ constexpr uint32_t make_idesc_major(int n, bool f16, bool a_mn, bool b_mn) {
+    return make_idesc(n, f16) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16);
 }
 
 __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accum) {

@@ -35,6 +35,12 @@ class ConvDesc(ctypes.Structure):
                 ("out16", c_void_p), ("in_dtype", c_int), ("max_ctas", c_int)]
 
 
+class GemmDesc(ctypes.Structure):
+    _fields_ = [("a", c_void_p), ("b", c_void_p), ("c", c_void_p), ("alpha", c_void_p), ("bias", c_void_p),
+                ("M", c_int), ("N", c_int), ("K", c_int), ("lda", c_int), ("ldb", c_int), ("ldc", c_int),
+                ("a_mn_major", c_int), ("b_mn_major", c_int)]
+
+
 class ProposalTargetCfg(ctypes.Structure):
     _fields_ = [("rois_per_image", c_int), ("fg_rois_per_image", c_int), ("fg_thresh", c_float),
                 ("bg_thresh_hi", c_float), ("bg_thresh_lo", c_float), ("bbox_means", c_float * 4),
@@ -59,6 +65,11 @@ _SIGS = {
     "sb_roi_align_pyramid_nhwc": (c_int, [ctypes.POINTER(c_void_p), ctypes.POINTER(c_int), ctypes.POINTER(c_int),
                                           c_int, c_float, c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int,
                                           c_void_p]),
+    "sb_roi_align_pyramid_nhwc_backward_workspace": (c_size_t, [c_int, ctypes.POINTER(c_int), ctypes.POINTER(c_int),
+                                                                 c_int]),
+    "sb_roi_align_pyramid_nhwc_backward": (c_int, [c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_int, c_int, c_int,
+                                                   ctypes.POINTER(c_int), ctypes.POINTER(c_int), ctypes.POINTER(c_void_p),
+                                                   c_void_p, c_size_t, c_void_p]),
     "sb_proposal_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "sb_proposal_layer": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, ctypes.POINTER(ProposalCfg),
                                   c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
@@ -79,6 +90,7 @@ _SIGS = {
     "sb_conv2d_simt": (c_int, [ctypes.POINTER(ConvDesc), c_void_p]),
     "sb_conv2d_tc": (c_int, [ctypes.POINTER(ConvDesc), c_void_p]),
     "sb_conv2d_tc_supported": (c_int, [ctypes.POINTER(ConvDesc)]),
+    "sb_gemm_tc": (c_int, [ctypes.POINTER(GemmDesc), c_void_p]),
     "sb_conv_trace_bytes": (c_size_t, [c_int]),
     "sb_conv_trace": (c_int, [c_void_p, c_int]),
     "sb_conv_trace_count": (c_int, []),
@@ -118,6 +130,13 @@ _SIGS = {
                             c_void_p]),
     "sb_rcnn_loss": (c_int, [c_void_p] * 14 + [c_int, c_int, c_int] + [c_void_p] * 8 + [c_void_p]),
     "sb_multitask_loss": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "sb_dropout": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "sb_box_tail_logits": (c_int, [c_void_p, c_int, c_int, c_int] + [c_void_p] * 9 + [c_void_p]),
+    "sb_box_tail_backward": (c_int, [c_void_p] * 4 + [c_int, c_int, c_int] + [c_void_p] * 10 + [c_void_p]),
+    "sb_dropout_backward_workspace": (c_size_t, [c_int, c_int]),
+    "sb_dropout_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_size_t, c_void_p]),
+    "sb_permute_pc_to_cp": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "sb_clip_gradient_workspace": (c_size_t, [c_int]),
     "sb_clip_gradient": (c_int, [ctypes.POINTER(c_void_p), ctypes.POINTER(c_size_t), c_int, c_float, c_void_p, c_size_t,
                                  c_void_p, c_void_p]),

@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import lib as _l
-from .lib import ConvDesc, ProposalCfg, check, ptr, stream_ptr
+from .lib import ConvDesc, GemmDesc, ProposalCfg, check, ptr, stream_ptr
 
 # constants of lib/model/utils/config.py that the hot path reads (SURVEY section 5)
 CFG = dict(
@@ -157,6 +157,60 @@ def roi_align_pyramid_nhwc(feats, im_h, rois, pooled, out=None, out_coff=0, roun
     check(L.sb_roi_align_pyramid_nhwc(fp, hs, ws_, C, float(im_h), ptr(_f32c(rois)), R, pooled, ptr(out),
                                       out.shape[3], out_coff, int(round_tf32), stream_ptr()),
           "sb_roi_align_pyramid_nhwc")
+    return out
+
+
+def roi_align_pyramid_nhwc_backward(top_grad, im_h, rois, feat_shapes, out_coff=0, grad_feats=None):
+    """adjoint of roi_align_pyramid_nhwc (deterministic, fixed-point accumulation): top_grad [R,P,P,ld] fp32 read at
+    channels [out_coff, out_coff + C); feat_shapes = 4 (N, H_l, W_l, C) of P2..P5 -> grad_feats, 4 fp32 NHWC tensors
+    (overwritten; allocated when not given)"""
+    L = _l.load()
+    assert top_grad.dtype == torch.float32 and top_grad.is_contiguous() and top_grad.dim() == 4
+    R, P = top_grad.shape[0], top_grad.shape[1]
+    N, C = int(feat_shapes[0][0]), int(feat_shapes[0][3])
+    dev = top_grad.device
+    if grad_feats is None:
+        grad_feats = [torch.empty(*[int(v) for v in s], dtype=torch.float32, device=dev) for s in feat_shapes]
+    for g, s in zip(grad_feats, feat_shapes):
+        assert g.dtype == torch.float32 and g.is_contiguous() and tuple(g.shape) == tuple(int(v) for v in s)
+    hs = (ctypes.c_int * 4)(*[int(s[1]) for s in feat_shapes])
+    ws_ = (ctypes.c_int * 4)(*[int(s[2]) for s in feat_shapes])
+    gp = (ctypes.c_void_p * 4)(*[g.data_ptr() for g in grad_feats])
+    nbytes = L.sb_roi_align_pyramid_nhwc_backward_workspace(N, hs, ws_, C)
+    ws = workspace(nbytes, dev, "roi_pyramid_bwd")
+    check(L.sb_roi_align_pyramid_nhwc_backward(ptr(top_grad), top_grad.shape[3], int(out_coff), C, float(im_h),
+                                               ptr(_f32c(rois)), R, P, N, hs, ws_, gp, ptr(ws), nbytes, stream_ptr()),
+          "sb_roi_align_pyramid_nhwc_backward")
+    return grad_feats
+
+
+# ------------------------------------------------------------------ GEMM ----
+def gemm(a, b, out, a_mn_major, b_mn_major, alpha=None, bias=None):
+    """out[m][n] = alpha * sum_k A(m,k) B(n,k) + bias[n] on the tensor cores (fp16 operands, fp32 accumulation).
+
+    a: fp16 [M, K] (a_mn_major False) or [K, M] (True, A read in place, no transposed copy); b likewise [N, K] or
+    [K, N]; out: fp32 [M, N].  Row-pitched views are fine (unit column stride, row strides multiples of 8).  alpha: fp32
+    DEVICE tensor of one element or None (1); bias: fp32 [N] or None."""
+    L = _l.load()
+    assert a.dtype == torch.float16 and b.dtype == torch.float16 and out.dtype == torch.float32
+    for t in (a, b, out):
+        assert t.is_cuda and t.dim() == 2 and t.stride(1) == 1, "gemm operands are 2-D with unit column stride"
+    M, N = out.shape
+    K = a.shape[0] if a_mn_major else a.shape[1]
+    assert tuple(a.shape) == ((K, M) if a_mn_major else (M, K)), "A shape"
+    assert tuple(b.shape) == ((K, N) if b_mn_major else (N, K)), "B shape"
+    if alpha is not None:
+        assert alpha.dtype == torch.float32 and alpha.numel() == 1 and alpha.is_cuda
+    if bias is not None:
+        assert bias.dtype == torch.float32 and bias.is_contiguous() and bias.numel() == N
+    d = GemmDesc()
+    d.a, d.b, d.c = a.data_ptr(), b.data_ptr(), out.data_ptr()
+    d.alpha = alpha.data_ptr() if alpha is not None else None
+    d.bias = bias.data_ptr() if bias is not None else None
+    d.M, d.N, d.K = M, N, K
+    d.lda, d.ldb, d.ldc = a.stride(0), b.stride(0), out.stride(0)
+    d.a_mn_major, d.b_mn_major = int(bool(a_mn_major)), int(bool(b_mn_major))
+    check(L.sb_gemm_tc(ctypes.byref(d), stream_ptr()), "sb_gemm_tc")
     return out
 
 

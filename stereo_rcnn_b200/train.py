@@ -173,3 +173,151 @@ def clip_gradient(grads, clip_norm):
     check(L.sb_clip_gradient(ptrs, counts, n, float(clip_norm), ptr(ws), nbytes, ptr(out), stream_ptr()),
           "sb_clip_gradient")
     return out
+
+
+# ---------------------------------------------------------------------------------------------- box-head training step
+# RCNN_top (Conv2d 512->2048 k7 s7 + ReLU + Dropout(0.2), Conv2d 2048->2048 k1 + ReLU + Dropout(0.2); resnet.py:256-263)
+# and the three tail linears (resnet.py:282-285), as stereo_rcnn.py:248-257 runs them in training.  fp16 engine only.
+# The forward reuses the engine's packed weights and conv kernels; the backward is sb_gemm_tc for the four products,
+# SIMT kernels for the tail, the dropout / ReLU masks and the device-chosen fp16 scaling, and the deterministic
+# pyramid RoIAlign adjoint into the feature gradients.  Stream ordered, no host reads: graph capturable.
+DROPOUT_KEEP_FROM = 858993460          # keep where the uint32 word >= 0.2 * 2^32 (nn.Dropout(p=0.2)), scale 1 / 0.8
+
+BOX_HEAD_PARAMS = ("RCNN_top.0.weight", "RCNN_top.0.bias", "RCNN_top.3.weight", "RCNN_top.3.bias",
+                   "RCNN_cls_score.weight", "RCNN_cls_score.bias", "RCNN_bbox_pred.weight", "RCNN_bbox_pred.bias",
+                   "RCNN_dim_orien_pred.weight", "RCNN_dim_orien_pred.bias")
+
+
+def box_head_param_shapes(n_classes=2):
+    """the reference's state_dict shapes of the box-head parameters, in BOX_HEAD_PARAMS order"""
+    nc = n_classes
+    return [(2048, 512, 7, 7), (2048,), (2048, 2048, 1, 1), (2048,), (nc, 2048), (nc,), (6 * nc, 2048), (6 * nc,),
+            (5 * nc, 2048), (5 * nc,)]
+
+
+def _need_fp16(eng):
+    if not getattr(eng, "half", False):
+        raise NotImplementedError("the box-head training step exists for the fp16 engine (precision='fp16') only")
+
+
+def _dropout(x, words, out32=None, out16=None):
+    L = _l.load()
+    R, C = x.shape
+    check(L.sb_dropout(ptr(x), ptr(_words(words)), R, C, ptr(out32), ptr(out16), stream_ptr()), "sb_dropout")
+
+
+def box_head_forward(eng, feats, B, rois_left, rois_right, im_h, drop_words):
+    """training forward of the box head (stereo_rcnn.py:248-257).  feats: {"p2".."p5": [2B,H,W,256] fp32 NHWC, left
+    images first} as the engine's trunk produces them; rois_* [R,5] (batch index first); drop_words = (w6, w7), two
+    int32 [R,2048] random-word tensors (train.random_words) for the dropouts after the two ReLUs of RCNN_top.
+    -> ctx: the tensors the forward consumed (pooled fp16, fc6 / fc7 ReLU outputs, fc6 after dropout fp16, fc7 after
+    dropout fp32, the words) and its outputs cls_score [R,nc] (logits), bbox_pred [R,6nc], dim_orien_pred [R,5nc]."""
+    _need_fp16(eng)
+    L = _l.load()
+    from . import ops
+    mk = ("p2", "p3", "p4", "p5")
+    fl, fr = [feats[k][:B] for k in mk], [feats[k][B:] for k in mk]
+    R = rois_left.shape[0]
+    dev = rois_left.device
+    w6, w7 = drop_words
+    assert w6.shape == (R, 2048) and w7.shape == (R, 2048)
+    pooled = torch.empty(R, 7, 7, 512, dtype=torch.float16, device=dev)
+    ops.roi_align_pyramid_nhwc(fl, im_h, rois_left, 7, out=pooled, out_coff=0, half=True)
+    ops.roi_align_pyramid_nhwc(fr, im_h, rois_right, 7, out=pooled, out_coff=256, half=True)
+    fc6 = eng._conv(pooled.view(R, 1, 1, 7 * 7 * 512), eng.p["RCNN_top.0"], relu=True, tag="top0").view(R, 2048)
+    fc6_drop = torch.empty(R, 2048, dtype=torch.float16, device=dev)
+    _dropout(fc6, w6, out16=fc6_drop)
+    fc7 = eng._conv(fc6_drop.view(R, 1, 1, 2048), eng.p["RCNN_top.3"], relu=True, tag="top3").view(R, 2048)
+    fc7_drop = torch.empty(R, 2048, dtype=torch.float32, device=dev)
+    _dropout(fc7, w7, out32=fc7_drop)
+    nc = eng.n_classes
+    cls = torch.empty(R, nc, dtype=torch.float32, device=dev)
+    bbox = torch.empty(R, 6 * nc, dtype=torch.float32, device=dev)
+    dim = torch.empty(R, 5 * nc, dtype=torch.float32, device=dev)
+    check(L.sb_box_tail_logits(ptr(fc7_drop), R, 2048, nc, *[ptr(t) for t in eng.fc], ptr(cls), ptr(bbox), ptr(dim),
+                               stream_ptr()), "sb_box_tail_logits")
+    return dict(pooled=pooled, fc6=fc6, fc6_drop=fc6_drop, fc7=fc7, fc7_drop=fc7_drop, words6=w6, words7=w7,
+                rois_left=rois_left, rois_right=rois_right, im_h=float(im_h), B=B,
+                feat_shapes=[tuple(f.shape) for f in fl], cls_score=cls, bbox_pred=bbox, dim_orien_pred=dim)
+
+
+def _dropout_backward(dy, y, words, db, tag):
+    """-> fp16 operand g * 2^e and the device scalar 2^-e (g = dy * mask * 1.25 * ReLU'); db written"""
+    L = _l.load()
+    R, C = dy.shape
+    nbytes = L.sb_dropout_backward_workspace(R, C)
+    ws = workspace(nbytes, dy.device, tag)
+    g16 = torch.empty(R, C, dtype=torch.float16, device=dy.device)
+    inv = torch.empty(1, dtype=torch.float32, device=dy.device)
+    check(L.sb_dropout_backward(ptr(dy), ptr(y), ptr(_words(words)), R, C, ptr(db), ptr(g16), ptr(inv), ptr(ws),
+                                nbytes, stream_ptr()), "sb_dropout_backward")
+    return g16, inv
+
+
+def box_head_backward(eng, ctx, d_cls_score, d_bbox_pred, d_dim_orien_pred, grads=None, feat_grads=None,
+                      stage_events=None):
+    """adjoint of box_head_forward.  d_* = d loss / d (cls_score, bbox_pred, dim_orien_pred), e.g. from rcnn_loss.
+    grads: optional {name: tensor} in the reference's state_dict shapes (BOX_HEAD_PARAMS; e.g. GradientBuckets views),
+    overwritten in place; feat_grads: optional {"left": [4 tensors], "right": [...]} fp32 NHWC [B,H_l,W_l,256].
+    stage_events: optional list; a (stage name, recorded CUDA event) pair is appended after each stage (per-stage
+    timing of eager runs).  -> (grads, feat_grads)"""
+    _need_fp16(eng)
+    L = _l.load()
+    from . import ops
+    R = ctx["pooled"].shape[0]
+    dev = ctx["pooled"].device
+    nc = eng.n_classes
+    if grads is None:
+        grads = {n: torch.empty(*s, dtype=torch.float32, device=dev)
+                 for n, s in zip(BOX_HEAD_PARAMS, box_head_param_shapes(nc))}
+    for n, s in zip(BOX_HEAD_PARAMS, box_head_param_shapes(nc)):
+        g = grads[n]
+        assert tuple(g.shape) == s and g.dtype == torch.float32 and g.is_contiguous(), n
+    def mark(name):
+        if stage_events is not None:
+            ev = torch.cuda.Event(enable_timing=True)
+            ev.record()
+            stage_events.append((name, ev))
+    mark("start")
+    # 1. tail: d_fc7 and the tail's weight / bias gradients (fixed-order sums over R)
+    d_fc7 = torch.empty(R, 2048, dtype=torch.float32, device=dev)
+    wc, _bc, wb, _bb, wd, _bd = eng.fc
+    check(L.sb_box_tail_backward(ptr(_f32c(d_cls_score)), ptr(_f32c(d_bbox_pred)), ptr(_f32c(d_dim_orien_pred)),
+                                 ptr(ctx["fc7_drop"]), R, 2048, nc, ptr(wc), ptr(wb), ptr(wd), ptr(d_fc7),
+                                 ptr(grads["RCNN_cls_score.weight"]), ptr(grads["RCNN_cls_score.bias"]),
+                                 ptr(grads["RCNN_bbox_pred.weight"]), ptr(grads["RCNN_bbox_pred.bias"]),
+                                 ptr(grads["RCNN_dim_orien_pred.weight"]), ptr(grads["RCNN_dim_orien_pred.bias"]),
+                                 stream_ptr()), "sb_box_tail_backward")
+    mark("tail backward")
+    # 2-3. fc7: mask / scale / convert, dW7 = g7^T fc6_drop, d_fc6 = g7 W7
+    g7, inv7 = _dropout_backward(d_fc7, ctx["fc7"], ctx["words7"], grads["RCNN_top.3.bias"], "box_bwd_fc7")
+    mark("mask/scale g7")
+    ops.gemm(g7, ctx["fc6_drop"], grads["RCNN_top.3.weight"].view(2048, 2048), True, True, alpha=inv7)
+    mark("dW7")
+    d_fc6 = torch.empty(R, 2048, dtype=torch.float32, device=dev)
+    ops.gemm(g7, eng.p["RCNN_top.3"].w16.view(2048, 2048), d_fc6, False, True, alpha=inv7)
+    mark("d_fc6")
+    # 4-5. fc6: mask / scale / convert, dW6 = g6^T pooled (packed (ph, pw, c) order, then one permute pass into
+    # [2048][512][7][7]), d_pooled = g6 W6
+    g6, inv6 = _dropout_backward(d_fc6, ctx["fc6"], ctx["words6"], grads["RCNN_top.0.bias"], "box_bwd_fc6")
+    mark("mask/scale g6")
+    dw6 = workspace(2048 * 25088 * 4, dev, "box_bwd_dw6")[:2048 * 25088 * 4].view(torch.float32).view(2048, 25088)
+    ops.gemm(g6, ctx["pooled"].view(R, 25088), dw6, True, True, alpha=inv6)
+    mark("dW6")
+    check(L.sb_permute_pc_to_cp(ptr(dw6), 2048, 49, 512, ptr(grads["RCNN_top.0.weight"]), stream_ptr()),
+          "sb_permute_pc_to_cp")
+    mark("dW6 permute")
+    d_pooled = torch.empty(R, 7, 7, 512, dtype=torch.float32, device=dev)
+    ops.gemm(g6, eng.p["RCNN_top.0"].w16.view(2048, 25088), d_pooled.view(R, 25088), False, True, alpha=inv6)
+    mark("d_pooled")
+    # 6. into the left / right feature pyramids
+    shapes = ctx["feat_shapes"]
+    if feat_grads is None:
+        feat_grads = {side: [torch.empty(*s, dtype=torch.float32, device=dev) for s in shapes]
+                      for side in ("left", "right")}
+    ops.roi_align_pyramid_nhwc_backward(d_pooled, ctx["im_h"], ctx["rois_left"], shapes, out_coff=0,
+                                        grad_feats=feat_grads["left"])
+    ops.roi_align_pyramid_nhwc_backward(d_pooled, ctx["im_h"], ctx["rois_right"], shapes, out_coff=256,
+                                        grad_feats=feat_grads["right"])
+    mark("RoIAlign backward L + R")
+    return grads, feat_grads
